@@ -3,6 +3,7 @@
 
   python bench.py [--config c2|c3|c4|c5] --gpus N --steps K --warmup W     (N>1: under torch.distributed.run, one rank/GPU)
   python bench.py --impl reference ...        (the CPU restatement of lamejs, oracle/, on the box's host cores)
+  python bench.py ... --dump-outputs DIR      (also writes the MP3 bytes of the last timed step, to compare two builds)
 
 Workloads (BASELINE.json configs, SURVEY.md 8(d)); c2 is the headline the metric is quoted on:
   c2  stereo 44.1 kHz 128 kbps, one 10 000-frame sine sweep per GPU                       (weak scaling)
@@ -39,6 +40,7 @@ CONFIGS = {
     "c5": (2, 44100, 128, 100, 1000, "burst", "strong", "BASELINE config #5 input (transient bursts, block switching) under CBR 128k (VBR is dead code in lamejs): 100 streams x 1000 frames"),
 }
 DISTINCT = 64      # c3-c5: this many distinct seeded streams, cycled (generation time; every stream is still encoded)
+DUMP_BYTES = 64 << 20   # --dump-outputs: at most this much float32 on disk
 # algorithmic bytes per frame x channel (SURVEY.md 8(d), DESIGN.md): groups of kernels, and the dominant single kernel
 ALGO_BYTES = {"filterbank_mdct": 6912, "psy": 3304, "quantizer": 5800}
 OUTER_BYTES_PER_GC = 2304 + 2304 + 1152 + 288 + 184 + 1152 + 288   # k_q_outer per granule-channel: xr, xrpow, lines, side info in; lines, side info out
@@ -186,6 +188,18 @@ def run_reference(args, rank, world):
     print(json.dumps(line))
 
 
+def dump_outputs(path, streams):
+    """Writes path/mp3_bytes.npy: the encoded bytes of every stream (torch uint8, streams x stream bytes) as float32.  Above
+    DUMP_BYTES, a fixed seeded sample of whole streams, kept in stream order."""
+    import torch
+    k = max(1, DUMP_BYTES // (4 * streams.shape[1]))
+    if streams.shape[0] > k:
+        idx = np.sort(np.random.default_rng(0).choice(streams.shape[0], k, replace=False))
+        streams = streams[torch.as_tensor(idx, device=streams.device)]
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "mp3_bytes.npy"), streams.cpu().numpy().astype(np.float32))
+
+
 def handle_api_numbers(M, L, dev_index):
     """The lamejs call pattern on the GPU: (a) ONE Mp3Encoder fed README-style 1152-sample encodeBuffer calls; (b) 256 live
     encoders advanced one 1152-sample call each per mp3b200_encode_batch launch."""
@@ -226,7 +240,11 @@ def main():
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--config", default="c2", choices=sorted(CONFIGS))
     ap.add_argument("--streams-per-gpu", type=int, default=1, help="c2 only: sweep streams per GPU")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the MP3 bytes of the last timed step to DIR/mp3_bytes.npy "
+                    "(float32, one row per stream, rank order; a seeded sample of streams above 64 MB)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -343,6 +361,13 @@ def main():
             coll_ms += ev_c0.elapsed_time(ev_c1)
         ktimes += tm
     launches = L.mp3b200_launch_count() - launches0
+    if args.dump_outputs and rank == 0:
+        if world == 1:
+            rows = d_out[:S * nbytes].view(S, nbytes)
+        else:
+            counts = [args.streams_per_gpu if cfg == "c2" else len(shard_streams(S_total, world, r)) for r in range(world)]
+            rows = torch.cat([g.view(S_max, nbytes)[:n] for g, n in zip(gather, counts)])
+        dump_outputs(args.dump_outputs, rows)
     own_ms = total_ms / args.steps
     t = torch.tensor([total_ms, -total_ms, coll_ms], dtype=torch.float64, device=dev)
     if world > 1:

@@ -1,12 +1,11 @@
 """The pin against the reference itself.  tests/golden/lamejs_golden.json holds SHA-256 / length / per-call sizes
-of the bytes REAL lamejs produced (unmodified /root/reference executed by Qt's QJSEngine, see tools/jsrun/ and
+of the bytes REAL lamejs produced (unmodified lamejs executed by Qt's QJSEngine, see tools/jsrun/ and
 tests/golden/make_lamejs_golden.py).  The oracle must reproduce every fixture it supports on CPU; the CUDA path must
-reproduce them through the C-ABI on the B200; and when the engine + /root/reference are present (this container, not
-the GPU box) a few randomly drawn inputs are pushed through lamejs live."""
+reproduce them through the C-ABI on the B200.  tests/golden/lamejs_seeded_golden.json (make_lamejs_seeded_golden.py)
+adds lamejs's bytes for seeded random configurations, for its three loaders, and its intermediates of one more input."""
 import hashlib
 import json
 import os
-import sys
 
 import numpy as np
 import pytest
@@ -14,10 +13,10 @@ import pytest
 from synth import make_signal
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-ROOT = os.path.dirname(HERE)
 _GOLD = json.load(open(os.path.join(HERE, "golden", "lamejs_golden.json")))
 FIX = _GOLD["cases"]
 TAPS = _GOLD["taps"]     # lamejs's own intermediates (SHA-256 per array): MDCT spectrum, masking, block types, quantised lines ...
+SEEDED = json.load(open(os.path.join(HERE, "golden", "lamejs_seeded_golden.json")))
 
 
 def _supported(oracle, c):
@@ -87,44 +86,24 @@ def test_gpu_matches_lamejs(name):
     _check(c, bytes(out), sizes)
 
 
-def _engine():
-    sys.path.insert(0, os.path.join(ROOT, "tools", "jsrun"))
-    import ref_lamejs
-    return ref_lamejs if ref_lamejs.available() else None
-
-
 @pytest.mark.parametrize("seed", range(6))
 def test_oracle_matches_live_lamejs_on_random_inputs(oracle, seed):
-    """Fresh inputs nobody has seen: random configuration, random signal kind, random chunking."""
-    R = _engine()
-    if R is None:
-        pytest.skip("no JS engine / reference here (GPU box)")
-    rng = np.random.default_rng(0xA11CE + seed)
-    ch = int(rng.integers(1, 3))
-    sr = int(rng.choice([32000, 44100, 48000]))
-    kbps = int(rng.choice([128, 160, 192, 224, 256, 320]))
-    kind = str(rng.choice(["noise", "white", "octave", "burst"]))
-    n = int(rng.integers(5, 40)) * 1152 + int(rng.integers(0, 1152))
-    chunk = [None, 1152, int(rng.integers(1, 4000))][int(rng.integers(0, 3))]
-    l, r = make_signal(kind, n, sr, 1000 + seed)
-    ref, ref_sizes, _ = R.encode(ch, sr, kbps, l, r, chunk=chunk)
-    got, sizes, _ = oracle.encode_stream(ch, sr, kbps, l, r if ch == 2 else None, chunk=chunk)
-    assert sizes == ref_sizes
-    assert got == ref
+    """Inputs drawn at random once: configuration, signal kind, length and chunking (make_lamejs_seeded_golden.py)."""
+    c = SEEDED["random_inputs"][str(seed)]
+    l, r = make_signal(c["kind"], c["samples"], c["samplerate"], c["seed"])
+    got, sizes, _ = oracle.encode_stream(c["channels"], c["samplerate"], c["kbps"], l, r if c["channels"] == 2 else None,
+                                         chunk=c["chunk"] or None)
+    _check(c, got, sizes)
 
 
-def test_loader_and_libm_independence():
-    """lame.all.js and the src/js modules give the same bytes; so does swapping the engine's libm for fdlibm."""
-    R = _engine()
-    if R is None:
-        pytest.skip("no JS engine / reference here (GPU box)")
-    l, r = make_signal("burst", 30 * 1152, 44100, 77)
-    a, _, _ = R.encode(2, 44100, 128, l, r)
-    b, _, _ = R.encode(2, 44100, 128, l, r, loader="modules")
-    assert a == b
-    if os.path.exists(os.path.join(ROOT, "tools", "jsrun", "fdlibm.js")):
-        c, _, _ = R.encode(2, 44100, 128, l, r, fdlibm=True)
-        assert a == c
+def test_loader_and_libm_independence(oracle):
+    """lame.all.js and the src/js modules gave the same bytes; so did swapping the engine's libm for fdlibm; the oracle
+    reproduces them."""
+    c = SEEDED["loaders"]
+    assert c["bundle"] == c["modules"] == c["fdlibm"]
+    l, r = make_signal(c["kind"], c["samples"], c["samplerate"], c["seed"])
+    data, _, _ = oracle.encode_stream(c["channels"], c["samplerate"], c["kbps"], l, r)
+    assert hashlib.sha256(data).hexdigest() == c["bundle"]
 
 
 def _tap_hash(a):
@@ -165,13 +144,10 @@ def test_gpu_intermediates_match_lamejs(name):
 
 
 def test_live_intermediates_on_a_random_input(oracle):
-    R = _engine()
-    if R is None:
-        pytest.skip("no JS engine / reference here (GPU box)")
-    l, r = make_signal("burst", 20 * 1152 + 3, 44100, 4242)
-    data, taps = R.encode_with_taps(2, 44100, 128, l, r)
-    ref, _, tr = oracle.encode_stream(2, 44100, 128, l, r, trace_frames=40)
-    assert data == ref
-    for k in ("xr", "en_l", "thm_l", "en_s", "thm_s", "blocktype", "l3_enc", "global_gain"):
-        assert _tap_hash(taps[k]) == _tap_hash(tr[k][:, :2, :2]), k
-    assert np.array_equal(taps["ath_adjust"], tr["ath_adjust"])
+    c = SEEDED["taps"]
+    l, r = make_signal(c["kind"], c["samples"], c["samplerate"], c["seed"])
+    data, _, tr = oracle.encode_stream(c["channels"], c["samplerate"], c["kbps"], l, r, trace_frames=40)
+    assert hashlib.sha256(data).hexdigest() == c["sha256"] and len(tr) == c["frames"]
+    for k, want in c["taps"].items():
+        a = tr[k] if k == "ath_adjust" else tr[k][:, :2, :2]
+        assert _tap_hash(a) == want, k

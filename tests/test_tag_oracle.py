@@ -1,11 +1,10 @@
 """SURVEY.md 8(f3), oracle side: music CRC / byte count kept by copy_buffer, the Xing / Info / LAME tag frame and the WAV
 header reader of oracle/lj_vbrtag.cpp against what REAL lamejs computed under the engine
-(tests/golden/lamejs_tag_golden.json, made by tests/golden/make_lamejs_tag_golden.py; live re-check when the engine and
-/root/reference are present)."""
+(tests/golden/lamejs_tag_golden.json, made by tests/golden/make_lamejs_tag_golden.py; seeded uniform-noise cases in
+tests/golden/lamejs_seeded_golden.json, made by tests/golden/make_lamejs_seeded_golden.py)."""
 import hashlib
 import json
 import os
-import sys
 
 import numpy as np
 import pytest
@@ -13,8 +12,8 @@ import pytest
 from synth import make_signal
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-ROOT = os.path.dirname(HERE)
 GOLD = json.load(open(os.path.join(HERE, "golden", "lamejs_tag_golden.json")))
+ENGINE = json.load(open(os.path.join(HERE, "golden", "lamejs_seeded_golden.json")))["engine"]
 
 # VBRTag.js:113-145: entries of crc16Lookup as printed in the reference, and the SHA-256 of all 256 (big-endian 16-bit)
 CRC_ROWS = {0: 0x0000, 1: 0xC0C1, 2: 0xC181, 3: 0x0140, 4: 0xC301, 8: 0xC601, 127: 0xE041, 128: 0xA001, 252: 0x4100, 253: 0x81C1, 254: 0x8081, 255: 0x4040}
@@ -142,32 +141,33 @@ def test_wav_header_matches_lamejs(oracle, name):
         assert oracle.wav_read_header(b) == want
 
 
+def _engine_pcm(c):
+    """Uniform PCM in [-20000, 20000), drawn as tests/golden/make_lamejs_seeded_golden.py drew it."""
+    rng = np.random.default_rng(c["pcm_seed"])
+    l = rng.integers(-20000, 20000, c["samples"]).astype(np.int16)
+    r = rng.integers(-20000, 20000, c["samples"]).astype(np.int16) if c["channels"] == 2 else None
+    return l, r
+
+
 def test_live_against_the_engine(oracle):
-    """When the engine and /root/reference are here (build container): fresh random cases pushed through lamejs now."""
-    sys.path.insert(0, os.path.join(ROOT, "tools", "jsrun"))
-    import ref_lamejs
-    if not ref_lamejs.available():
-        pytest.skip("no JavaScript engine / reference in this environment")
-    import tag_probe
-    rng = np.random.default_rng(int.from_bytes(os.urandom(4), "little"))
-    for _ in range(2):
-        ch = int(rng.integers(1, 3))
-        sr, kbps = [(48000, 192), (32000, 96), (44100, 160), (24000, 48), (22050, 64)][int(rng.integers(0, 5))]
-        n = int(rng.integers(5, 30)) * 1152 + int(rng.integers(0, 1152))
-        l = rng.integers(-20000, 20000, n).astype(np.int16)
-        r = rng.integers(-20000, 20000, n).astype(np.int16) if ch == 2 else None
-        chunk = int(rng.integers(500, 6000))
-        js, crc, nb = tag_probe.hot_path_crc(ch, sr, kbps, l, r, chunk=chunk)
+    """Cases drawn at random once (configuration, length, chunking, full-band PCM) and run through lamejs: hot-path bytes,
+    music CRC and byte count, and the tag frame."""
+    assert len(ENGINE) >= 8
+    for c in ENGINE:
+        ch, sr, kbps, n, chunk = c["channels"], c["samplerate"], c["kbps"], c["samples"], c["chunk"]
+        l, r = _engine_pcm(c)
         enc = oracle.OracleEncoder(ch, sr, kbps)
         out = bytearray()
         for i in range(0, n, chunk):
             out += enc.encode_buffer(l[i:i + chunk], None if r is None else r[i:i + chunk])
         out += enc.flush()
-        assert bytes(out) == js and enc.music_crc() == crc and enc.bytes_written() == nb, (ch, sr, kbps, n, chunk)
-        o = tag_probe.tagged(ch, sr, kbps, l, r, chunk=chunk)
+        assert hashlib.sha256(bytes(out)).hexdigest() == c["sha256"], (ch, sr, kbps, n, chunk)
+        assert enc.music_crc() == c["music_crc"] and enc.bytes_written() == c["bytes_written"], (ch, sr, kbps, n, chunk)
+        enc.close()
         _, _, info = oracle.encode_stream_tagged(ch, sr, kbps, l, r, chunk=chunk)
-        assert info["tag_on"] == o["write_tag"] and info["music_crc"] == o["crc"] and info["frames"] == o["frames"]
+        assert info["tag_on"] == c["write_tag"] and info["music_crc"] == c["tag_crc"] and info["frames"] == c["frames"]
         if info["tag_on"]:
-            t, _ = _js_view(info["tag"], o["tag"], o["sideinfo_len"])
-            k = o["sideinfo_len"] + 154
-            assert t[:k] == o["tag"][:k], (ch, sr, kbps, n, chunk)
+            js = bytes.fromhex(c["tag"])
+            t, _ = _js_view(info["tag"], js, c["sideinfo_len"])
+            k = c["sideinfo_len"] + 154
+            assert len(js) == k and t[:k] == js, (ch, sr, kbps, n, chunk)
